@@ -53,6 +53,9 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--dump-ops", default="", help="write per-op CUDA-event timings (JSON lines)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the UNet output of the last timed step as DIR/sample.npy (float32; "
+                         "sample_rank<r>.npy per rank when --gpus > 1)")
     ap.add_argument("--no-extras", action="store_true",
                     help="skip gpu_library_baseline / config4 / config2_sdxl (profiling runs)")
     return ap.parse_args()
@@ -157,7 +160,7 @@ def cross_dim(args):
 
 
 # ------------------------------------------------------------------------------------------------
-def cpu_reference_run(args, steps, warmup, budget_s):
+def cpu_reference_run(args, steps, warmup):
     """The reference's CPU path for this workload = plain eager PyTorch fp32 (every sfast op falls
     back to aten on CPU: /root/reference/src/sfast/csrc/operators/cublas/cublas_gemm.cpp:705-710,
     /root/reference/src/sfast/triton/torch_ops.py:116-126), run on the oracle restatement of the
@@ -177,23 +180,18 @@ def cpu_reference_run(args, steps, warmup, budget_s):
                                    "time_ids": torch.tensor([[1024., 1024, 0, 0, 1024, 1024]] * nb)}
     times = []
     with torch.no_grad():
-        t0 = time.perf_counter()
-        m(s, torch.tensor(999.0), e, **kw)
-        t_warm = time.perf_counter() - t0
-        # the requested warm-up and step counts, cut only if they would exceed the time budget
-        n_warm = max(1, min(warmup, int(0.3 * budget_s / max(t_warm, 1e-3))))
-        for _ in range(n_warm - 1):
+        for _ in range(warmup):
             m(s, torch.tensor(999.0), e, **kw)
-        n = max(1, min(steps, int(0.7 * budget_s / max(t_warm, 1e-3))))
-        for i in range(n):
+        for i in range(steps):
             t0 = time.perf_counter()
-            m(s, torch.tensor(999.0 - 50 * i), e, **kw)
+            out = m(s, torch.tensor(999.0 - 50 * i), e, **kw)
             times.append(time.perf_counter() - t0)
     times.sort()
     med = times[len(times) // 2]
-    return {"value": nb / med, "ms_per_step": med * 1e3, "steps": n, "warmup": n_warm, "cores": cores,
-            "sample": f"{n} timed fp32 eager forward(s) of {nb} {args.model} latent(s) "
-                      f"4x{args.size}x{args.size} (the same batch as one GPU rank) after {n_warm} warm-up(s), "
+    return {"value": nb / med, "ms_per_step": med * 1e3, "steps": steps, "warmup": warmup, "cores": cores,
+            "sample_out": out.sample,
+            "sample": f"{steps} timed fp32 eager forward(s) of {nb} {args.model} latent(s) "
+                      f"4x{args.size}x{args.size} (the same batch as one GPU rank) after {warmup} warm-up(s), "
                       f"{cores} threads, median"}
 
 
@@ -204,7 +202,9 @@ def run_reference(args, rank):
     if rank != 0:
         return
     world = args.gpus
-    r = cpu_reference_run(args, args.steps, args.warmup, budget_s=170.0)
+    r = cpu_reference_run(args, args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"sample": r["sample_out"]})
     total = args.global_batch if args.global_batch else args.batch * world
     line = {
         "impl": "reference", "metric": METRIC, "value": r["value"], "unit": UNIT,
@@ -297,10 +297,15 @@ def run_b200(args, rank, world, local):
         return ms, clocks
 
     # --- device-resident arm: inputs already in HBM; per step = static-buffer copies + graph replay
+    last = {}
+
     def step_dev(i):
-        unet(dev_s[i % n_var], tsteps[i % 20], dev_e[i % n_var], **kw)
+        last["sample"] = unet(dev_s[i % n_var], tsteps[i % 20], dev_e[i % n_var], **kw).sample
 
     ms_dev, clocks = timed(step_dev, args.steps, max(args.warmup, 3))
+    if args.dump_outputs:
+        # copied before the next arm reuses the graph's static output buffer
+        outputs = {"sample" if world == 1 else f"sample_rank{rank}": last["sample"].float().cpu()}
 
     # --- end-to-end arm: pinned host inputs -> H2D -> public API call -> D2H of the result
     def step_e2e(i):
@@ -310,6 +315,8 @@ def run_b200(args, rank, world, local):
         host_out.copy_(out, non_blocking=True)
 
     ms_e2e, _ = timed(step_e2e, args.steps, max(args.warmup, 3))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, budget=(64 << 20) // world)
 
     weight_gb = sum(int(torch.Size(sh).numel()) for sh in param_shapes(spec).values()) * 2 / 1e9
     flops_per_step = plan.flops()
@@ -342,7 +349,7 @@ def run_b200(args, rank, world, local):
         extras["text_encoder"] = text_encoder_bench(dev)
     cpu_base = None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
-        r = cpu_reference_run(args, steps=2, warmup=1, budget_s=25.0)
+        r = cpu_reference_run(args, steps=2, warmup=1)
         cpu_base = {"value": r["value"], "unit": UNIT, "cores": r["cores"], "kind": "port",
                     "sample": r["sample"]}
     if rank != 0:
@@ -366,6 +373,23 @@ def run_b200(args, rank, world, local):
         **extras,
     }
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(dirname, arrays, budget=64 << 20):
+    """Write each tensor as DIR/<name>.npy in float32, all together within `budget` bytes.  A tensor
+    over its share is replaced by a fixed seeded sample: its flat elements at the indices stored
+    beside it as DIR/<name>_index.npy (float64), so that two builds still compare element for element."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    share = budget // len(arrays)
+    for name, t in arrays.items():
+        a = t.numpy().astype(np.float32)
+        if a.nbytes > share:
+            n = (share - 4096) // 12  # a float32 value and a float64 index per kept element, headers
+            idx = np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))
+            np.save(os.path.join(dirname, f"{name}_index.npy"), idx.astype(np.float64))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(dirname, f"{name}.npy"), a)
 
 
 def family_rates(plan):

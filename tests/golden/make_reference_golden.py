@@ -15,10 +15,13 @@ code: (1) the script must run under `python -O` so the wrappers' `assert input.d
 (`copy_func(..., name=f'{kernel.__name__}_{act.__name__}')`, group_norm.py:87-96) -- the lookup
 falls back to the single function the source defines.
 
-Cases: the reference self-test configuration (group_norm.py:481-527: randn(2, 320, 32, 32) fp16,
-G = 32, randn affine, eps 1e-5, NCHW and channels_last, with and without SiLU), UNet-shaped
-extras (1280 channels at 8x8, a large-mean input, an outlier channel), and LayerNorm on the
-self-test's data recipe (layer_norm.py:406-438: x = -2.3 + 0.5 randn, rand affine) at UNet widths.
+Cases: reference_inputs.norm_cases() -- the reference self-test configuration (group_norm.py:481-527:
+randn(2, 320, 32, 32) fp16, G = 32, randn affine, eps 1e-5, NCHW and channels_last, with and without
+SiLU), UNet-shaped extras (1280 channels at 8x8, a large-mean input, an outlier channel), and
+LayerNorm on the self-test's data recipe (layer_norm.py:406-438: x = -2.3 + 0.5 randn, rand affine)
+at UNet widths.  The inputs are not stored (the test rebuilds them from the same seed); of each
+output the fixture keeps the GroupNorm statistics whole, reference_inputs.SAMPLES sampled elements
+of each GroupNorm output and 32 sampled rows of each LayerNorm output, which keeps it small.
 
 Run from the repo root (about 5 minutes):   python -O tests/golden/make_reference_golden.py
 """
@@ -27,9 +30,12 @@ import os
 import sys
 import types
 
-os.environ["TRITON_INTERPRET"] = "1"
+import torch
 
-import torch  # noqa: E402
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from golden import reference_inputs as ri  # noqa: E402
+
+REF_ROWS = 32  # LayerNorm output rows kept per case
 
 REF = "/root/reference/src/sfast"
 
@@ -37,6 +43,7 @@ REF = "/root/reference/src/sfast"
 def _load_reference_kernels():
     if __debug__:
         raise SystemExit("run with `python -O` (the reference wrappers assert a CUDA device)")
+    os.environ["TRITON_INTERPRET"] = "1"
     from triton.runtime import interpreter as ti
 
     def compile_and_exec(self, tree):
@@ -72,48 +79,33 @@ def main():
            "reference_files": ["triton/ops/group_norm.py", "triton/ops/layer_norm.py",
                                "triton/ops/activation.py", "triton/ops/utils.py"],
            "group_norm": [], "layer_norm": []}
-    g = torch.Generator().manual_seed(20260923)
-
-    def randn(*s):
-        return torch.randn(*s, generator=g)
-
-    gn_cases = [
-        # (tag, shape, transform of x)
-        ("selftest_2x320x32x32", (2, 320, 32, 32), None),
-        ("unet_2x1280x8x8", (2, 1280, 8, 8), None),
-        ("large_mean_1x320x16x16", (1, 320, 16, 16), "mean50"),
-        ("outlier_channel_1x640x8x8", (1, 640, 8, 8), "outlier"),
-    ]
-    for tag, shape, tf in gn_cases:
-        x = randn(*shape)
-        if tf == "mean50":
-            x = x + 50.0
-        elif tf == "outlier":
-            x[:, 7] *= 100.0
-        x = x.half()
-        w, b = randn(shape[1]).half(), randn(shape[1]).half()
-        case = {"tag": tag, "x": x, "weight": w, "bias": b, "groups": 32, "eps": 1e-5}
+    gn_cases, ln_cases = ri.norm_cases()
+    for i, inp in enumerate(gn_cases):
+        tag, x, w, b = inp["tag"], inp["x"], inp["weight"], inp["bias"]
+        idx = ri.sample_index(x.numel(), seed=i).long()
+        case = {"tag": tag, "groups": inp["groups"], "eps": inp["eps"], "idx": idx.int(),
+                "input_check": ri.input_check(x, w, b)}
         xcl = x.contiguous(memory_format=torch.channels_last)
         for silu, fn in ((False, gn.group_norm_forward), (True, gn.group_norm_silu_forward)):
             key = "silu" if silu else "plain"
             if tag.startswith("selftest"):
-                case["y_nchw_" + key] = fn(x, 32, w, b, 1e-5)[0].contiguous()
+                case["y_nchw_" + key] = fn(x, 32, w, b, 1e-5)[0].flatten()[idx]
             y, mean, rstd = fn(xcl, 32, w, b, 1e-5)
             assert y.is_contiguous(memory_format=torch.channels_last)
-            case["y_nhwc_" + key] = y.contiguous()  # stored in NCHW order, values of the NHWC kernel
+            # NCHW flat indices into the values of the NHWC kernel
+            case["y_nhwc_" + key] = y.contiguous().flatten()[idx]
             case["mean_" + key], case["rstd_" + key] = mean, rstd
         out["group_norm"].append(case)
         print("group_norm", tag, "done", flush=True)
 
-    for tag, (m, n) in (("selftest_recipe_257x1280", (257, 1280)), ("tokens_300x320", (300, 320)),
-                        ("tokens_64x640", (64, 640))):
-        weight = torch.rand(n, generator=g).half()
-        bias = torch.rand(n, generator=g).half()
-        x = (-2.3 + 0.5 * randn(m, n)).half()
+    for i, inp in enumerate(ln_cases):
+        x, weight, bias, n = inp["x"], inp["weight"], inp["bias"], inp["x"].shape[1]
         y = ln.LayerNorm.forward(types.SimpleNamespace(save_for_backward=lambda *a: None), x, (n,),
                                  weight, bias, 1e-5)
-        out["layer_norm"].append({"tag": tag, "x": x, "weight": weight, "bias": bias, "eps": 1e-5, "y": y})
-        print("layer_norm", tag, "done", flush=True)
+        rows = ri.sample_index(x.shape[0], seed=100 + i, count=REF_ROWS)
+        out["layer_norm"].append({"tag": inp["tag"], "eps": inp["eps"], "rows": rows, "y": y[rows.long()],
+                                  "input_check": ri.input_check(x, weight, bias)})
+        print("layer_norm", inp["tag"], "done", flush=True)
 
     path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_triton_norms.pt")
     torch.save(out, path)

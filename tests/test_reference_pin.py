@@ -1,8 +1,9 @@
 """Pins against outputs of the REFERENCE's own kernels.
 
-tests/golden/ref_triton_norms.pt holds what /root/reference/src/sfast/triton/ops/group_norm.py and
-layer_norm.py (unmodified, imported from /root/reference) computed under Triton's interpreter in
-the build container -- see tests/golden/make_reference_golden.py.  Rows a4 (GroupNorm / GroupNorm +
+tests/golden/ref_triton_norms.pt holds what the reference's triton/ops/group_norm.py and
+layer_norm.py (unmodified) computed under Triton's interpreter -- see
+tests/golden/make_reference_golden.py; the inputs are rebuilt from their seed by
+tests/golden/reference_inputs.py and the outputs are sampled.  Rows a4 (GroupNorm / GroupNorm +
 SiLU) and a9 (LayerNorm) of SURVEY.md section 8 are therefore pinned to reference-run vectors
 (zero-mean cases at the reference's own 1e-2; the large-mean case with the reference's own fp16
 arithmetic error added, see _stat_slack):
@@ -22,13 +23,35 @@ import os
 import pytest
 import torch
 
+from golden import reference_inputs as ri
 from oracle import ops_oracle as oo
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "ref_triton_norms.pt")
+GOLDEN_GEGLU = os.path.join(os.path.dirname(__file__), "golden", "ref_cutlass_geglu.pt")
+
+
+def _check_inputs(case, *tensors):
+    """The rebuilt inputs are the ones the reference was run on."""
+    for got, want in zip(ri.input_check(*tensors), case["input_check"], strict=True):
+        assert torch.equal(got, want), "reference_inputs no longer rebuilds the fixture's inputs"
 
 
 def _fx():
-    return torch.load(GOLDEN)
+    """The fixture with each case's inputs (x, weight, bias) rebuilt from their seed."""
+    fx = torch.load(GOLDEN)
+    gn, ln = ri.norm_cases()
+    for case, inp in zip(fx["group_norm"] + fx["layer_norm"], gn + ln, strict=True):
+        assert case["tag"] == inp["tag"]
+        _check_inputs(case, inp["x"], inp["weight"], inp["bias"])
+        case.update(x=inp["x"], weight=inp["weight"], bias=inp["bias"])
+    return fx
+
+
+def _at(y, case):
+    """The elements (GroupNorm, NCHW flat indices) or rows (LayerNorm) the fixture kept of y."""
+    if "idx" in case:
+        return y.flatten()[case["idx"].long().to(y.device)]
+    return y[case["rows"].long().to(y.device)]
 
 
 def _close(got, ref, rtol=1e-2, atol=1e-2):
@@ -78,10 +101,10 @@ def test_ops_oracle_group_norm_matches_reference_triton_outputs(silu):
     for case in _fx()["group_norm"]:
         got = oo.group_norm(case["x"], case["groups"], case["weight"], case["bias"], case["eps"], silu)
         slack = _stat_slack(case, key)
-        _close(got, case["y_nhwc_" + key], atol=1e-2 + slack)
-        _close(_with_reference_stats(case, key, silu), case["y_nhwc_" + key], atol=1e-2 + slack)
+        _close(_at(got, case), case["y_nhwc_" + key], atol=1e-2 + slack)
+        _close(_at(_with_reference_stats(case, key, silu), case), case["y_nhwc_" + key], atol=1e-2 + slack)
         if "y_nchw_" + key in case:
-            _close(got, case["y_nchw_" + key], atol=1e-2 + slack)
+            _close(_at(got, case), case["y_nchw_" + key], atol=1e-2 + slack)
         # the statistics themselves (the reference stores them in fp16)
         n, c = case["x"].shape[:2]
         xf = case["x"].float().reshape(n, case["groups"], -1)
@@ -93,7 +116,7 @@ def test_ops_oracle_group_norm_matches_reference_triton_outputs(silu):
 def test_ops_oracle_layer_norm_matches_reference_triton_outputs():
     for case in _fx()["layer_norm"]:
         got = oo.layer_norm(case["x"], case["weight"], case["bias"], case["eps"])
-        _close(got, case["y"], rtol=0, atol=1e-2)
+        _close(_at(got, case), case["y"], rtol=0, atol=1e-2)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -120,7 +143,7 @@ def test_cuda_group_norm_matches_reference_triton_outputs(silu, fused):
         for op in gops:
             op.launch(torch.cuda.current_stream().cuda_stream)
         torch.cuda.synchronize()
-        _close(yb.permute(0, 3, 1, 2), case["y_nhwc_" + key], atol=1e-2 + _stat_slack(case, key))
+        _close(_at(yb.permute(0, 3, 1, 2), case), case["y_nhwc_" + key], atol=1e-2 + _stat_slack(case, key))
         # and tightly against the fp32-statistics oracle (what the reference approximates)
         want = oo.group_norm(case["x"], case["groups"], case["weight"], case["bias"], case["eps"], silu)
         _close(yb.permute(0, 3, 1, 2), want, rtol=4e-3, atol=4e-3)
@@ -140,10 +163,13 @@ def test_cuda_layer_norm_and_folded_layer_norm_match_reference_triton_outputs():
         ops.ln_op("ln", lib, x=x, y=y, rows=rows, c=c, gamma=gamma, beta=beta, eps=case["eps"],
                   dt=torch.float16).launch(st)
         torch.cuda.synchronize()
-        _close(y, case["y"], rtol=0, atol=1e-2)
+        _close(_at(y, case), case["y"], rtol=0, atol=1e-2)
+        # and the whole output tightly against the fp32 oracle
+        _close(y, oo.layer_norm(case["x"], case["weight"], case["bias"], case["eps"]), rtol=4e-3, atol=4e-3)
         # (2) the product path: LayerNorm folded into the consuming tcgen05 GEMM.  Row statistics as
         # the producer epilogue would leave them (sum, sum of squares of the stored fp16 row); the
-        # expected result is the REFERENCE LayerNorm output pushed through the same linear in fp32.
+        # expected result is the REFERENCE LayerNorm output pushed through the same linear in fp32,
+        # on the rows the fixture kept.
         torch.manual_seed(1)
         n_out = 320
         w = (torch.randn(n_out, c, device="cuda") / math.sqrt(c)).half()
@@ -158,29 +184,24 @@ def test_cuda_layer_norm_and_folded_layer_norm_match_reference_triton_outputs():
         torch.cuda.synchronize()
         ref = case["y"].cuda().float() @ w.float().t() + b
         # the reference LN output is itself fp16-rounded: allow its quantisation through the GEMM
-        _close(out, ref, rtol=1e-2, atol=2e-2)
+        _close(_at(out, case), ref, rtol=1e-2, atol=2e-2)
+        # and every row against the fp16-rounded oracle LayerNorm pushed through the same linear
+        want = oo.layer_norm(x, gamma, beta, case["eps"]).float() @ w.float().t() + b
+        _close(out, want, rtol=1e-2, atol=2e-2)
 
 
 # ------------------------------------------------------------------------------------------------
-# Row a7: Linear + GEGLU pinned against the reference's own CUTLASS kernel RUN ON THE B200
-# (/root/reference/src/sfast/csrc/operators/cutlass/cutlass_dual_linear_kernel.cu, compiled from its
-# own source by oracle/build_ref.sh into oracle/_ref/ -- the git-ignored .so travels with the
-# snapshot).
-_REF_GEGLU = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref",
-                          "libsfast_ref_geglu.so")
-
-
-def _ref_geglu_op():
-    if not os.path.exists(_REF_GEGLU):
-        pytest.skip("oracle/_ref/libsfast_ref_geglu.so not built (run oracle/build_ref.sh where "
-                    "/root/reference exists)")
-    torch.ops.load_library(_REF_GEGLU)
-    return torch.ops.sfast_ref.linear_geglu
+# Row a7: Linear + GEGLU pinned against the reference's own CUTLASS kernel run on a B200
+# (the reference's csrc/operators/cutlass/cutlass_dual_linear_kernel.cu, compiled from its own
+# source by oracle/build_ref.sh); tests/golden/ref_cutlass_geglu.pt holds its outputs -- see
+# tests/golden/make_reference_geglu_golden.py.
+def _geglu_fx():
+    return torch.load(GOLDEN_GEGLU)
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype", [torch.float16, torch.bfloat16])
-@pytest.mark.parametrize("shape", [(4608, 320, 1280), (1152, 640, 2560), (300, 1280, 5120), (18432, 320, 1280)])
+@pytest.mark.parametrize("shape", ri.GEGLU_SHAPES)
 def test_cuda_geglu_matches_reference_cutlass_kernel(dtype, shape):
     """UNet GEGLU sizes (the reference's benchmark test uses in_features 320 / 640 -> 1280 / 2560,
     tests/operators/test_cutlass_dual_linear.py:59-72) at the reference's tolerance 2e-2: the
@@ -188,15 +209,15 @@ def test_cuda_geglu_matches_reference_cutlass_kernel(dtype, shape):
     reference accumulates in fp16 / bf16 and uses the tanh GELU under torch's default flags
     (cutlass_dual_linear_kernel.cu:391-393,509-514); the CUDA path accumulates in fp32 with erf."""
     from sfast_b200 import _lib, ops
-    ref_op = _ref_geglu_op()
+    case = next(c for c in _geglu_fx()["unet"]
+                if c["dtype"] == str(dtype).replace("torch.", "") and tuple(c["shape"]) == shape)
     lib = _lib.lib()
     m, k, inner = shape
-    torch.manual_seed(m + k)
-    x = torch.randn(m, k, device="cuda").to(dtype)
-    w = (torch.randn(2 * inner, k, device="cuda") / math.sqrt(k)).to(dtype)
-    b = (torch.randn(2 * inner, device="cuda") * 0.1).to(dtype)
-    ref = ref_op(x, w, b)
-    assert ref.shape == (m, inner) and ref.dtype == dtype
+    x, w, b = ri.geglu_inputs(dtype, shape)
+    _check_inputs(case, x, w, b)
+    x, w, b = x.cuda(), w.cuda(), b.cuda()
+    ref = case["y"].cuda()
+    assert ref.dtype == dtype
     want = oo.linear_geglu(x, w, b)
     wp, bp, _ = ops.pack_geglu(w, b.float(), dtype)
     out = torch.zeros(m, inner, device="cuda", dtype=dtype)
@@ -205,22 +226,20 @@ def test_cuda_geglu_matches_reference_cutlass_kernel(dtype, shape):
                 splits=1).launch(torch.cuda.current_stream().cuda_stream)
     torch.cuda.synchronize()
     tol = 2e-2 if dtype == torch.float16 else 6e-2   # the bf16 reference accumulates in bf16
-    _close(want, ref, rtol=tol, atol=tol)             # oracle  vs reference-run
-    _close(out, ref, rtol=tol, atol=tol)              # product vs reference-run
+    _close(_at(want, case), ref, rtol=tol, atol=tol)  # oracle  vs reference-run
+    _close(_at(out, case), ref, rtol=tol, atol=tol)   # product vs reference-run
     _close(out, want, rtol=1e-2, atol=1e-2)           # product vs oracle (fp32 truth), tighter
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("bias", [False, True])
 def test_reference_cutlass_kernel_on_its_own_test_configuration(bias):
-    """The reference's own small-shape test (tests/operators/test_cutlass_dual_linear.py:42-56) run
-    against the oracle -- checks the oracle's chunk order / GELU against the reference binary."""
-    ref_op = _ref_geglu_op()
-    for n in (4, 16):
-        for cin in (8, 16):
-            for cout in (8, 16):
-                torch.manual_seed(n * 100 + cin * 10 + cout)
-                proj = torch.nn.Linear(cin, 2 * cout, bias=bias).cuda().half()
-                x = torch.randn(n, cin, device="cuda").half()
-                got = ref_op(x, proj.weight, proj.bias)
-                _close(oo.linear_geglu(x, proj.weight, proj.bias), got, rtol=2e-2, atol=2e-2)
+    """The reference's own small-shape test (tests/operators/test_cutlass_dual_linear.py:42-56,
+    n in (4, 16), in / out features in (8, 16)) run against the oracle -- checks the oracle's chunk
+    order / GELU against the reference binary's outputs."""
+    cases = [c for c in _geglu_fx()["own_config"] if (c["bias"] is not None) == bias]
+    assert len(cases) == 8
+    for c in cases:
+        x, wt = c["x"].cuda(), c["weight"].cuda()
+        bs = c["bias"].cuda() if bias else None
+        _close(oo.linear_geglu(x, wt, bs), c["y"], rtol=2e-2, atol=2e-2)
